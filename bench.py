@@ -2,6 +2,7 @@
 """bench.py — env-steps/s of the fused GEM step on B200 (BASELINE.json metric), with roofline + CPU baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config pmsm|pmsm_64k|fin_sc_pmsm|scim|eesm|mixed] [--envs-per-gpu E]
+                    [--dump-outputs DIR]
 
 Default workload (BASELINE.json metric / configs[1] at the size the metric is quoted on): Cont-CC-PMSM-v0, RK4 (one step per
 tau = 1e-4), 2^20 envs per GPU, synthetic U(-1,1)^3 actions, Wiener references, in-kernel auto-reset; weak scaling: every rank steps its
@@ -42,6 +43,7 @@ if ROOT not in sys.path:
 METRIC = "env-steps/sec at N=2^20 PMSM, 1/2/4/8 GPU; HBM GB/s vs roofline"
 UNIT = "env-steps/s"
 ROLL_MAX = 32  # steps per fused launch (bounds the size of the recorded trajectory: 32 x 72 MB at N = 2^20)
+DUMP_ENVS = 1 << 16  # envs per array written by --dump-outputs: a fixed sample keeps the default 2^20-env workload at ~5 MB
 
 # BASELINE.json configs; n_* feed the algorithmic-bytes bookkeeping of SURVEY.md §8(d)
 CONFIGS = {
@@ -315,6 +317,24 @@ class Workload:
         self.env.close()
 
 
+def dump_outputs(wl, K, out_dir):
+    """Write what the timed path returned for its last step — obs, reference, reward and terminated of the last of the K fused steps — as
+    <out_dir>/<name>.npy in float32 (mixed batch: <type>_<name>.npy), for a fixed sample of DUMP_ENVS envs drawn with seed 0 (sorted env
+    indices), so that two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    last = (K - 1) % ROLL_MAX  # slot of the last step in the last fused launch (Workload.steps issues launches of ROLL_MAX steps first)
+    for i, (s, outs) in enumerate(zip(wl.sims, wl.outs)):
+        idx = np.sort(np.random.default_rng(0).choice(s.n, size=min(s.n, DUMP_ENVS), replace=False))
+        sel = wl.torch.as_tensor(idx, device=wl.dev)
+        prefix = f"{wl.c['types'][i]}_" if wl.mixed else ""
+        for name, t in zip(("obs", "reference", "reward", "terminated"), outs):
+            if name == "reference" and not s.n_ref:
+                continue
+            np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), t[last].index_select(0, sel).float().cpu().numpy())
+
+
 def gate(torch):
     """Keep the GPU busy for ~0.15 ms right before a timed region starts: the start event is recorded BEHIND this spin kernel, so the host
     has queued the timed launches by the time the event fires and the event-to-event time is device time of the K steps only — no host
@@ -408,7 +428,10 @@ def main():
     ap.add_argument("--envs-per-gpu", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the brief timings of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's outputs (a fixed sample of envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -449,6 +472,8 @@ def main():
         sampler.wait_first()
         sampler.mark()
     ms, launches, t_wall = time_rollout(wl, K, W, barrier, torch)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, K, args.dump_outputs)
     # the same K steps with only the LAST step's outputs written (what an open-loop consumer of the final state pays)
     wl.steps(3, every=0)
     barrier()

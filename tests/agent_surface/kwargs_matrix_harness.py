@@ -4,7 +4,8 @@ with the unmodified reference (`--impl reference`) and once with this repo's hos
 (`--impl b200`, which also derives the C-ABI config).  Each case is a source snippet evaluated with `gem` bound to the respective
 package, so both sides see literally the same user code.  Prints {case: {"verdict", "summary"}}; the summaries (names, limits, nominal
 state, spaces, tau, motor / load parameters, supply, reward weights / range / bias, constraint list, generator margins) must agree.
-No stepping, no GPU.  Container-only: needs /root/reference."""
+No stepping, no GPU.  `--impl reference` needs the reference checkout (REF); its output is stored in
+tests/golden/agent_surface/kwargs_matrix_reference.npz (tests/golden/make_agent_surface_golden.py)."""
 import json
 import sys
 import warnings

@@ -2,7 +2,9 @@
 computes actions from fixed observations, once against the unmodified reference and once against this package aliased as
 `gym_electric_motor` (tests/agent_surface/harness.py).  Everything the agent reads — classes and isinstance relations, env class per
 id, spaces, names, limits, nominal values, parameters, tau, index attributes, transformation helpers — must lead to the same actions.
-Container-only (needs /root/reference); the portable part of the surface is pinned through env_table.json in test_host_envs.py."""
+The tests that run the reference's own example code need the reference checkout (agent_surface/harness.py:REF) and skip without it; the
+kwargs matrix and the INTEGRATION.md stub compare against the reference's side stored under tests/golden/agent_surface/
+(tests/golden/make_agent_surface_golden.py), and the portable part of the surface is pinned through env_table.json in test_host_envs.py."""
 import json
 import os
 import subprocess
@@ -13,7 +15,11 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 HARNESS = os.path.join(HERE, "agent_surface", "harness.py")
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/examples/classic_controllers"), reason="needs the reference checkout")
+GOLDEN = os.path.join(HERE, "golden", "agent_surface")
+sys.path.insert(0, os.path.join(HERE, "agent_surface"))
+from harness import REF  # noqa: E402
+
+needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples", "classic_controllers")), reason="needs the reference checkout")
 
 
 SCRATCH = __import__("tempfile").mkdtemp(prefix="gemb200_agent_surface_")  # tutorial code creates files under the cwd: keep them out of the repo
@@ -25,6 +31,7 @@ def _run(impl):
     return json.loads(out.stdout.strip().splitlines()[-1])
 
 
+@needs_reference
 def test_reference_example_agent_reads_the_same_surface():
     ref, mine = _run("reference"), _run("b200")
     assert sorted(ref) == sorted(mine) and len(ref) == 54
@@ -47,6 +54,7 @@ def test_reference_example_agent_reads_the_same_surface():
             assert r["error"] == m["error"], (env_id, r["error"], m["error"])
 
 
+@needs_reference
 def test_reference_example_scripts_build_the_same_environments():
     """examples/environment_features/*.py, examples/classic_controllers/*_example.py and the gem.make cells of the RL / MPC notebooks,
     unmodified, up to `env = gem.make(...)` (tests/agent_surface/examples_harness.py), against the reference and against this package:
@@ -75,6 +83,7 @@ def test_reference_example_scripts_build_the_same_environments():
     assert compared >= 11
 
 
+@needs_reference
 def test_gem_cookbook_cells_build_the_same_environment():
     """examples/environment_features/GEM_cookbook.ipynb, cell by cell (tests/agent_surface/cookbook_harness.py)"""
     out = subprocess.run([sys.executable, os.path.join(HERE, "agent_surface", "cookbook_harness.py")], capture_output=True, text=True, timeout=600, cwd=SCRATCH)
@@ -90,16 +99,31 @@ def test_gem_cookbook_cells_build_the_same_environment():
 
 
 def test_integration_md_binding_stub_reaches_gemb200_create():
-    """the ctypes stub of INTEGRATION.md section B, run verbatim against a reference SCMLSystem (tests/agent_surface/integration_stub_harness.py)"""
+    """the ctypes stub of INTEGRATION.md section B, run verbatim against this package's SCMLSystem (tests/agent_surface/integration_stub_harness.py),
+    which must present every value the stub reads exactly as the reference's SCMLSystem did (tests/golden/agent_surface/integration_stub_reference.json)"""
     import torch
 
-    out = subprocess.run([sys.executable, os.path.join(HERE, "agent_surface", "integration_stub_harness.py")], capture_output=True, text=True, timeout=600, cwd=SCRATCH)
+    out = subprocess.run([sys.executable, os.path.join(HERE, "agent_surface", "integration_stub_harness.py"), "--impl", "b200"], capture_output=True, text=True,
+                         timeout=600, cwd=SCRATCH)
     assert out.returncode == 0, out.stderr[-2000:]
-    verdict = out.stdout.strip().splitlines()[-1]
+    res = json.loads(out.stdout.strip().splitlines()[-1])
+    with open(os.path.join(GOLDEN, "integration_stub_reference.json")) as f:
+        assert res["reads"] == json.load(f)
+    verdict = res["verdict"]
     if torch.cuda.is_available():
         assert verdict.startswith("created"), verdict
     else:
         assert verdict.startswith("GemB200Error") and "rc=-2" in verdict, verdict   # GEMB200_E_CUDA: validation passed, no device
+
+
+def _reference_kwargs_matrix():
+    """the reference's side of kwargs_matrix_harness.py; trajectories hold the state rows `rows` (a fixed sample) of `n_states`"""
+    z = np.load(os.path.join(GOLDEN, "kwargs_matrix_reference.npz"))
+    ref = json.loads(str(z["cases"]))
+    for case, rec in ref.items():
+        if rec["trajectory"] is not None:
+            rec["trajectory"].update(rows=z[f"rows/{case}"].tolist(), states=z[f"states/{case}"])
+    return ref
 
 
 def test_user_kwargs_matrix_builds_identical_environments():
@@ -109,13 +133,11 @@ def test_user_kwargs_matrix_builds_identical_environments():
     must be equal.  One documented exception: a ConstReferenceGenerator's `reference_names` is the bare string in the reference
     (const_reference_generator.py:24), which a MultipleReferenceGenerator then extends its list with character by character; here it is
     the one-element list every other generator has."""
-    res = {}
-    for impl in ("reference", "b200"):
-        out = subprocess.run([sys.executable, os.path.join(HERE, "agent_surface", "kwargs_matrix_harness.py"), "--impl", impl], capture_output=True, text=True,
-                             timeout=600, cwd=SCRATCH)
-        assert out.returncode == 0, out.stderr[-2000:]
-        res[impl] = json.loads(out.stdout.strip().splitlines()[-1])
-    ref, mine = res["reference"], res["b200"]
+    ref = _reference_kwargs_matrix()
+    out = subprocess.run([sys.executable, os.path.join(HERE, "agent_surface", "kwargs_matrix_harness.py"), "--impl", "b200"], capture_output=True, text=True,
+                         timeout=600, cwd=SCRATCH)
+    assert out.returncode == 0, out.stderr[-2000:]
+    mine = json.loads(out.stdout.strip().splitlines()[-1])
     assert sorted(ref) == sorted(mine) and len(ref) >= 166
     compared_trajectories = compared_rewards = refused = long_runs = terminations = 0
     for case in sorted(ref):
@@ -147,7 +169,7 @@ def test_user_kwargs_matrix_builds_identical_environments():
         assert (ta is None) == (tb is None), case
         if ta is None:
             continue  # random initial state / supply phase / state noise: RNG streams differ by design
-        assert len(ta["states"]) == len(tb["states"]) and len(ta["states"]) >= 2, case
+        assert ta["n_states"] == len(tb["states"]) and ta["n_states"] >= 2, case
         tol = {"ScipyOdeSolver": 1e-9, "EulerSolver": 1e-9, "ScipyOdeIntSolver": 1e-6, "ScipySolveIvpSolver": 1e-4}[ta["solver"]]
         reset_rows, row = {0}, 0
         for flag in ta["terminated"]:
@@ -155,10 +177,11 @@ def test_user_kwargs_matrix_builds_identical_environments():
             if flag and len(ta["terminated"]) > 5:
                 row += 1
                 reset_rows.add(row)
-        for i, (x, y) in enumerate(zip(ta["states"], tb["states"])):
+        for i, x in zip(ta["rows"], ta["states"]):
             if case == "cossin_remove" and i in reset_rows:
                 continue  # documented deviation at reset (DESIGN.md §7)
-            assert np.max(np.abs(np.asarray(x) - np.asarray(y))) < tol, (case, i, x, y)
+            y = tb["states"][i]
+            assert np.max(np.abs(x - np.asarray(y))) < tol, (case, i, x, y)
         long_runs += len(ta["terminated"]) > 5
         terminations += sum(ta["terminated"])
         assert ta["terminated"] == tb["terminated"], case

@@ -1,9 +1,13 @@
-"""bench.py contract pieces that run without a GPU: the `--impl reference` arm (CPU oracle port on the host cores) prints one JSON line
-with the keys the driver reads; under a multi-rank launch only rank 0 prints; the GPU arm refuses to run without a device."""
+"""bench.py contract pieces: the `--impl reference` arm (CPU oracle port on the host cores) prints one JSON line with the keys a
+consumer of the line reads; under a multi-rank launch only rank 0 prints; the GPU arm refuses to run without a device; on a GPU,
+`--dump-outputs` writes the timed path's last outputs, identical from run to run."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASELINE = json.load(open(os.path.join(ROOT, "BASELINE.json"))) if os.path.exists(os.path.join(ROOT, "BASELINE.json")) else None
@@ -46,3 +50,21 @@ def test_gpu_arm_refuses_without_a_device():
         return
     out = _run(["--steps", "2", "--warmup", "1"])
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_path_are_reproducible(tmp_path):
+    """--dump-outputs writes the last of the --steps timed steps as float32 .npy files; the same arguments give the same arrays"""
+    lines = []
+    for run in ("a", "b"):
+        out = _run(["--gpus", "1", "--steps", "37", "--warmup", "3", "--envs-per-gpu", "4096", "--no-extra", "--no-cpu-baseline",
+                    "--dump-outputs", str(tmp_path / run)])
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines.append(json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1]))
+    assert lines[0]["steps"] == 37 and lines[0]["gpu_launches"] == 2  # 32 + 5 fused steps
+    shapes = {"obs": (4096, 14), "reference": (4096, 2), "reward": (4096,), "terminated": (4096,)}
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(f"{k}.npy" for k in shapes)
+    for name, shape in shapes.items():
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float32 and a.shape == shape and np.isfinite(a).all()
+        assert np.array_equal(a, b), name
